@@ -31,6 +31,10 @@ Legs (timed regions run in C, mrbayes_b200/host/mb200_host_loop.c, a plain clien
 
 --impl reference times the reference's own CPU path on this arm's config (one serial process per
 analysis: N processes under torchrun, rank 0 runs them all).
+
+--dump-outputs DIR writes what the value and e2e legs computed in their last timed step (every chain's lnL
+in every generation, the chains' state after it, the coordinator's heats and swap counters) as
+DIR/<name>.npy; the inputs are seeded, so two builds can be compared output for output (see dump_outputs).
 """
 from __future__ import annotations
 
@@ -260,8 +264,9 @@ class Job:
         self.cur_lnl = self.lnl0.copy()
         self.cur_lnpr = self.lnpr0.copy()
 
-    def run(self, hl, mode, order, swap_freq=1):
-        """-> (wall seconds, device ms, swaps accepted) for the generations in `order`."""
+    def run(self, hl, mode, order, swap_freq=1, trace=None):
+        """-> (wall seconds, device ms, swaps accepted) for the generations in `order`; `trace`, if given, a float64
+        array [len(order)][n_local] that receives every chain's lnL in every generation."""
         arr = (C.c_int * len(order))(*order)
         sums = (C.c_double * 2)()
         nacc = C.c_longlong(0)
@@ -270,7 +275,8 @@ class Job:
                                     self.c_accept.ctypes.data_as(C.POINTER(C.c_ubyte)),
                                     self.c_lnprior.ctypes.data_as(C.POINTER(C.c_double)), arr, len(order), swap_freq,
                                     self.cur_lnl.ctypes.data_as(C.POINTER(C.c_double)),
-                                    self.cur_lnpr.ctypes.data_as(C.POINTER(C.c_double)), sums, C.byref(nacc))
+                                    self.cur_lnpr.ctypes.data_as(C.POINTER(C.c_double)), sums, C.byref(nacc),
+                                    None if trace is None else trace.ctypes.data_as(C.POINTER(C.c_double)))
         if rc != 0:
             raise RuntimeError(f"mb200_host_mc3_loop failed with code {rc}")
         return sums[0], sums[1], nacc.value
@@ -311,7 +317,7 @@ def load_host_loop():
     hl.mb200_host_mc3_loop.argtypes = [C.c_void_p, C.POINTER(C.c_int), C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p),
                                        C.POINTER(C.c_int), C.c_int, C.POINTER(C.c_ubyte), C.POINTER(C.c_double),
                                        C.POINTER(C.c_int), C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double),
-                                       C.POINTER(C.c_double), C.POINTER(C.c_longlong)]
+                                       C.POINTER(C.c_double), C.POINTER(C.c_longlong), C.POINTER(C.c_double)]
     hl.mb200_host_generation_loop.restype = C.c_double
     hl.mb200_host_replay_loop.restype = C.c_double
     return hl
@@ -453,18 +459,20 @@ def reference_sample(name: str, n_procs: int, seed0: int, ngen_scale: float = 1.
     ngen = max(1, int(ngen * ngen_scale))
     with tempfile.TemporaryDirectory() as td:
         tmp = Path(td)
+        # the processes run in the temporary directory and see short relative names only: MrBayes refuses file names
+        # longer than 99 characters
+        data = tmp / f"{name}.nex"
         if name in SYNTH:
-            data = tmp / f"{name}.nex"
             write_synthetic_nexus(name, data)
         else:
-            data = REF_DATA / ("primates.nex" if name.startswith("primates") else f"{name}.nex")
+            data.symlink_to(REF_DATA / ("primates.nex" if name.startswith("primates") else f"{name}.nex"))
         procs = []
         t0 = time.perf_counter()
         for i in range(n_procs):
             nex = tmp / f"p{i}.nex"
-            nex.write_text(reference_commands(name, data, nruns, nchains, ngen, seed0 + i, tmp / f"p{i}"))
+            nex.write_text(reference_commands(name, Path(data.name), nruns, nchains, ngen, seed0 + i, Path(f"p{i}")))
             env = dict(os.environ, MB200_MODE="cpu", MB200_REPORT=str(tmp / f"p{i}.json"))
-            procs.append(subprocess.Popen([str(REF_BIN), str(nex)], env=env, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL))
+            procs.append(subprocess.Popen([str(REF_BIN), nex.name], cwd=tmp, env=env, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL))
         for p in procs:
             p.wait()
         wall = time.perf_counter() - t0
@@ -722,18 +730,23 @@ def bench_engine(args):
             i.synchronize()
         torch.cuda.synchronize()
 
-    def run_steps(mode, n_steps, timed):
-        """n_steps steps of G generations each, L2 flushed before every step; -> (device ms, wall s, updates, swaps)."""
+    def run_steps(mode, n_steps, timed, record=None):
+        """n_steps steps of G generations each, L2 flushed before every step; -> (device ms, wall s, updates, swaps).
+        `record`, if given, a dict that receives what the last step computed: every chain's lnL in every generation
+        and the chains' current lnL / log prior after it."""
         ms_tot = wall_tot = upd = 0.0
         nacc = 0
         g0 = 0
-        for _ in range(n_steps):
+        for s in range(n_steps):
             order = [(g0 + g) % cycle_len for g in range(G)]
             g0 = (g0 + G) % cycle_len
             if timed:
                 flush.zero_()
                 torch.cuda.synchronize()
-            wall, ms, acc = job.run(hl, mode, order)
+            trace = np.zeros((G, job.n_local)) if record is not None and s == n_steps - 1 else None
+            wall, ms, acc = job.run(hl, mode, order, trace=trace)
+            if trace is not None:
+                record.update(lnl=trace, current_lnl=job.cur_lnl.copy(), current_lnprior=job.cur_lnpr.copy())
             ms_tot += ms; wall_tot += wall; nacc += acc
             upd += float(sum(job.updates_per_step[i] for i in order))
         # return to the cycle start so that the next leg replays the same generations
@@ -754,7 +767,8 @@ def bench_engine(args):
     coll0 = mc.collectives()
     barrier()
     t_clock0 = time.perf_counter()
-    ms_value, wall_value, updates, swaps_acc = run_steps(1, K, True)
+    out_value, out_e2e = {}, {}
+    ms_value, wall_value, updates, swaps_acc = run_steps(1, K, True, out_value if args.dump_outputs else None)
     barrier()
     launches = sum(i.launch_count() for i in job.insts) - launches0
     collectives = mc.collectives() - coll0
@@ -771,11 +785,17 @@ def bench_engine(args):
 
     # ---- e2e: host structs through the C-ABI ----
     barrier()
-    ms_e2e_dev, wall_e2e, updates_e2e, _ = run_steps(0, K, True)
+    mc3_state = {"chain_id": np.array([mc.chain_id(g) for g in range(job.runs * job.chains)], np.float64),
+                 "swap_info": mc.swap_info().astype(np.float64)} if args.dump_outputs else {}
+    ms_e2e_dev, wall_e2e, updates_e2e, _ = run_steps(0, K, True, out_e2e if args.dump_outputs else None)
     barrier()
     t_clock1 = time.perf_counter()
     if rank == 0:
         sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, rank if world > 1 else None,
+                     {**{f"value_{k}": v for k, v in out_value.items()}, **{f"e2e_{k}": v for k, v in out_e2e.items()},
+                      **{f"mc3_{k}": v for k, v in mc3_state.items()}})
 
     # ---- reduce over ranks: MAX time, SUM work ----
     vals = torch.tensor([ms_value, wall_value * 1e3, wall_e2e * 1e3], dtype=torch.float64, device=dev)
@@ -854,6 +874,23 @@ def bench_engine(args):
         dist.destroy_process_group()
 
 
+def dump_outputs(out_dir, rank, arrays, limit=64 << 20):
+    """Writes what the timed legs computed in their last step as out_dir/<name>.npy (float64; `rank` prefixes the
+    names of a multi-process run), so that two builds can be compared output for output on identical inputs:
+      value_lnl / e2e_lnl                 [G][chains]: lnL of every local chain's proposal in every generation of the
+                                          last timed step (resident descriptors / host structs through the C-ABI)
+      value_current_lnl, _current_lnprior [chains]: each chain's state after that step (likewise e2e_*)
+      mc3_chain_id, mc3_swap_info         the coordinator's heat assignment and swap counters after the value leg"""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > limit:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes (limit {limit})")
+    for k, a in arrays.items():
+        np.save(d / (k if rank is None else f"rank{rank}_{k}"), a)
+
+
 class pack_bytes:
     """Size of the packed job a generation ships host->device (header + DevEval + rates/frequencies + branch
     list + node records).  Small jobs ride in the kernel parameter block, i.e. inside the launch."""
@@ -879,7 +916,13 @@ def main():
                     help="N=1 default workload only: large synthetic configs reported under other_workloads ('' = none)")
     ap.add_argument("--no-extras", action="store_true", help="skip many_analyses / other_workloads")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed legs computed in their last step to DIR/<name>.npy (engine arm only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the engine arm's outputs")
     if args.impl == "reference":
         bench_reference(args)
     else:

@@ -168,6 +168,7 @@ double mb200_host_replay_loop (const int *instances, int replicas, const int *ba
  *   lnprior          lnprior[i * n_local + c]: log prior of that proposal
  *   cur_lnl/cur_lnpr in: state before the first generation; out: state after the last
  *   sums             out: [2] wall-clock seconds, device milliseconds (events on the first partition's stream)
+ *   lnl_trace        out, may be NULL: lnl_trace[g * n_local + c] = lnL of local chain c's proposal in generation g
  * Returns 0 or a negative error code.
  */
 #include "mb200_mc3.h"
@@ -175,7 +176,8 @@ double mb200_host_replay_loop (const int *instances, int replicas, const int *ba
 int mb200_host_mc3_loop (mb200_mc3 *mc, const int *parts, int n_parts, int n_local, int mode,
                          const mb200_evaluation *const *steps, const int *batches, int cycle,
                          const unsigned char *accept, const double *lnprior, const int *order, int n_generations,
-                         int swap_freq, double *cur_lnl, double *cur_lnpr, double *sums, long long *swaps_accepted)
+                         int swap_freq, double *cur_lnl, double *cur_lnpr, double *sums, long long *swaps_accepted,
+                         double *lnl_trace)
 {
     struct timespec t0, t1;
     cudaEvent_t evA = NULL, evB = NULL;
@@ -234,6 +236,8 @@ int mb200_host_mc3_loop (mb200_mc3 *mc, const int *parts, int n_parts, int n_loc
                 lnl_new[c] += lnl_p[c];
             }
         if (rc != 0) break;
+        if (lnl_trace)
+            for (c = 0; c < n_local; c++) lnl_trace[(size_t) g * n_local + c] = lnl_new[c];
         /* accept / reject (the reference: r = exp (T * (lnL' - lnL) + T * (lnPr' - lnPr) + proposal ratio),
            src/mcmc.c:16865-16890; here the outcome is part of the pre-generated proposal cycle, because a
            rejected proposal's index flips are baked into the next step's evaluation) */

@@ -28,19 +28,30 @@ BIN = ROOT / "oracle" / "_ref" / "mb_b200"
 BIN_BATCHED = ROOT / "oracle" / "_ref" / "mb_b200_batched"     # the same objects with the patched RunChain (oracle/patch_runchain.py)
 CMD = ROOT / "tests" / "golden" / "cmd"
 
-needs_harness = pytest.mark.skipif(not BIN.exists(), reason="oracle/_ref/mb_b200 not built (needs /root/reference at build time)")
+needs_harness = pytest.mark.skipif(not BIN.exists(), reason="oracle/_ref/mb_b200 not built (needs the reference sources at build time)")
+
+
+def run_mb(binary: Path, nex: Path, env, timeout=900):
+    """Runs a harness binary on `nex` from the directory `nex` is in.  MrBayes refuses file names longer than 99 characters,
+    so the program sees short names relative to that directory only: the command files' output prefixes are bare names, and
+    `oracle` there links to the repository's oracle/ for their `execute oracle/_ref/data/...` lines."""
+    link = nex.parent / "oracle"
+    if not link.is_symlink():
+        link.symlink_to(ROOT / "oracle", target_is_directory=True)
+    return subprocess.run([str(binary), nex.name], cwd=nex.parent, env=env, stdout=subprocess.PIPE, stderr=subprocess.PIPE,
+                          text=True, timeout=timeout)
 
 
 def run_harness(tmp_path: Path, stem: str, ngen: int, mode: str, via: str = "seam", extra_env=None, timeout=900, binary: Path = BIN, tag: str = ""):
     key = f"{stem}.{mode}.{via}" if not tag else "r" + tag.replace(".", "_")     # MrBayes limits file name lengths to 100 characters
     nex = tmp_path / f"{key}.nex"
     prefix = tmp_path / (f"out_{stem}_{mode}_{via}" if not tag else "o" + tag.replace(".", "_"))
-    text = (CMD / f"{stem}.nex").read_text().replace("NGEN", str(ngen)).replace("OUTPREFIX", str(prefix))
+    text = (CMD / f"{stem}.nex").read_text().replace("NGEN", str(ngen)).replace("OUTPREFIX", prefix.name)
     nex.write_text(text)
     report = tmp_path / f"{key}.json"
     env = dict(os.environ, MB200_MODE=mode, MB200_REPORT=str(report), MB200_VIA=via)
     env.update(extra_env or {})
-    p = subprocess.run([str(binary), str(nex)], cwd=ROOT, env=env, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=timeout)
+    p = run_mb(binary, nex, env, timeout)
     assert p.returncode == 0, p.stdout[-2000:] + p.stderr[-2000:]
     assert report.exists(), p.stdout[-2000:] + p.stderr[-2000:]
     rep = json.loads(report.read_text().strip().splitlines()[-1])
@@ -120,11 +131,11 @@ def _run_inline(tmp_path, binary, mode, data, cmds, ngen, tag, env=None):
     d.mkdir()
     nex = d / "r.nex"
     nex.write_text(f"set autoclose=yes nowarn=yes seed=99 swapseed=99;\nexecute oracle/_ref/data/{data};\n{cmds}\n"
-                   f"mcmc nruns=2 nchains=3 ngen={ngen} printfreq=100000 samplefreq=25 diagnfreq=100000 filename={d}/o;\nquit;\n")
+                   f"mcmc nruns=2 nchains=3 ngen={ngen} printfreq=100000 samplefreq=25 diagnfreq=100000 filename=o;\nquit;\n")
     report = d / "r.json"
     e = dict(os.environ, MB200_MODE=mode, MB200_BATCH="1", MB200_REPORT=str(report))
     e.update(env or {})
-    p = subprocess.run([str(binary), str(nex)], cwd=ROOT, env=e, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=900)
+    p = run_mb(binary, nex, e)
     assert p.returncode == 0, p.stdout[-2000:] + p.stderr[-2000:]
     rep = json.loads(report.read_text().strip().splitlines()[-1])
     rep["samples"] = {f.name: "\n".join(l for l in f.read_text().splitlines() if "ID:" not in l)
@@ -152,10 +163,10 @@ def test_chain_batched_generations_with_other_chain_layouts(tmp_path, mc):
         d.mkdir()
         nex = d / "r.nex"
         nex.write_text(f"set autoclose=yes nowarn=yes seed=99 swapseed=99;\nexecute oracle/_ref/data/primates.nex;\nlset nst=6 rates=gamma;\n"
-                       f"mcmc {mc} printfreq=100000 samplefreq=25 diagnfreq=100000 filename={d}/o;\nquit;\n")
+                       f"mcmc {mc} printfreq=100000 samplefreq=25 diagnfreq=100000 filename=o;\nquit;\n")
         report = d / "r.json"
         e = dict(os.environ, MB200_MODE=mode, MB200_BATCH="1", MB200_REPORT=str(report))
-        p = subprocess.run([str(binary), str(nex)], cwd=ROOT, env=e, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=900)
+        p = run_mb(binary, nex, e)
         assert p.returncode == 0, p.stdout[-2000:] + p.stderr[-2000:]
         rep = json.loads(report.read_text().strip().splitlines()[-1])
         rep["samples"] = {f.name: "\n".join(l for l in f.read_text().splitlines() if "ID:" not in l)
@@ -177,13 +188,13 @@ def _lnl_columns(rep_stdout):
 
 def _run_printing(tmp_path, stem, ngen, env, tag, mode="oracle"):
     nex = tmp_path / f"r{tag}.nex"
-    text = (CMD / f"{stem}.nex").read_text().replace("NGEN", str(ngen)).replace("OUTPREFIX", str(tmp_path / f"o{tag}")) \
+    text = (CMD / f"{stem}.nex").read_text().replace("NGEN", str(ngen)).replace("OUTPREFIX", f"o{tag}") \
                                           .replace("printfreq=100000", "printfreq=1")
     nex.write_text(text)
     report = tmp_path / f"r{tag}.json"
     e = dict(os.environ, MB200_MODE=mode, MB200_BATCH="1", MB200_REPORT=str(report))
     e.update(env)
-    p = subprocess.run([str(BIN_BATCHED), str(nex)], cwd=ROOT, env=e, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=900)
+    p = run_mb(BIN_BATCHED, nex, e)
     assert p.returncode == 0, p.stdout[-2000:] + p.stderr[-2000:]
     return json.loads(report.read_text().strip().splitlines()[-1]), _lnl_columns(p.stdout)
 
@@ -295,11 +306,11 @@ MODEL_SWEEP = [
 def _run_sweep_case(tmp_path, data, cmds, ngen, env):
     nex = tmp_path / "sweep.nex"
     nex.write_text(f"set autoclose=yes nowarn=yes seed=99 swapseed=99;\nexecute oracle/_ref/data/{data};\n{cmds}\n"
-                   f"mcmc nruns=1 nchains=2 ngen={ngen} printfreq=100000 samplefreq=50 diagnfreq=100000 filename={tmp_path}/o;\nquit;\n")
+                   f"mcmc nruns=1 nchains=2 ngen={ngen} printfreq=100000 samplefreq=50 diagnfreq=100000 filename=o;\nquit;\n")
     report = tmp_path / "sweep.json"
     e = dict(os.environ, MB200_MODE="shadow", MB200_REPORT=str(report))
     e.update(env)
-    p = subprocess.run([str(BIN_SCALAR), str(nex)], cwd=ROOT, env=e, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=900)
+    p = run_mb(BIN_SCALAR, nex, e)
     assert p.returncode == 0, p.stdout[-2000:] + p.stderr[-2000:]
     return json.loads(report.read_text().strip().splitlines()[-1])
 
@@ -322,15 +333,15 @@ def _run_session(tmp_path, binary, mode, tag, env=None):
     d.mkdir()
     nex = d / "r.nex"
     nex.write_text("set autoclose=yes nowarn=yes seed=99 swapseed=99;\nexecute oracle/_ref/data/replicase.nex;\nlset nucmodel=codon;\n"
-                   f"mcmc nruns=1 nchains=2 ngen=40 printfreq=100000 samplefreq=20 diagnfreq=100000 filename={d}/a;\n"
+                   "mcmc nruns=1 nchains=2 ngen=40 printfreq=100000 samplefreq=20 diagnfreq=100000 filename=a;\n"
                    "lset nucmodel=4by4 nst=6 rates=gamma ngammacat=6;\n"
-                   f"mcmc nruns=1 nchains=3 ngen=60 printfreq=100000 samplefreq=20 diagnfreq=100000 filename={d}/b;\n"
+                   "mcmc nruns=1 nchains=3 ngen=60 printfreq=100000 samplefreq=20 diagnfreq=100000 filename=b;\n"
                    "lset nucmodel=codon omegavar=ny98;\n"
-                   f"mcmc nruns=1 nchains=2 ngen=40 printfreq=100000 samplefreq=20 diagnfreq=100000 filename={d}/c;\nquit;\n")
+                   "mcmc nruns=1 nchains=2 ngen=40 printfreq=100000 samplefreq=20 diagnfreq=100000 filename=c;\nquit;\n")
     report = d / "r.json"
     e = dict(os.environ, MB200_MODE=mode, MB200_BATCH="1", MB200_REPORT=str(report))
     e.update(env or {})
-    p = subprocess.run([str(binary), str(nex)], cwd=ROOT, env=e, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=900)
+    p = run_mb(binary, nex, e)
     assert p.returncode == 0, p.stdout[-2000:] + p.stderr[-2000:]
     rep = json.loads(report.read_text().strip().splitlines()[-1])
     rep["samples"] = {f.name: "\n".join(l for l in f.read_text().splitlines() if "ID:" not in l)
@@ -387,10 +398,10 @@ def test_function_pointer_forms_drive_like_the_seam_loop_over_models(tmp_path, d
         d.mkdir()
         nex = d / "r.nex"
         nex.write_text(f"set autoclose=yes nowarn=yes seed=99 swapseed=99;\nexecute oracle/_ref/data/{data};\n{cmds}\n"
-                       f"mcmc nruns=1 nchains=2 ngen=100 printfreq=100000 samplefreq=25 diagnfreq=100000 filename={d}/o;\nquit;\n")
+                       f"mcmc nruns=1 nchains=2 ngen=100 printfreq=100000 samplefreq=25 diagnfreq=100000 filename=o;\nquit;\n")
         report = d / "r.json"
         e = dict(os.environ, MB200_MODE="oracle", MB200_VIA=via, MB200_MULTIPART="0", MB200_EIGEN="host", MB200_REPORT=str(report))
-        p = subprocess.run([str(BIN_SCALAR), str(nex)], cwd=ROOT, env=e, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=900)
+        p = run_mb(BIN_SCALAR, nex, e)
         assert p.returncode == 0, p.stdout[-2000:] + p.stderr[-2000:]
         rep = json.loads(report.read_text().strip().splitlines()[-1])
         rep["samples"] = {f.name: "\n".join(l for l in f.read_text().splitlines() if "ID:" not in l)
@@ -571,11 +582,11 @@ def test_chain_batched_launches_equal_per_chain_launches_over_data_sets(tmp_path
         d.mkdir()
         nex = d / "r.nex"
         nex.write_text(f"set autoclose=yes nowarn=yes seed=99 swapseed=99;\nexecute oracle/_ref/data/{data};\n{cmds}\n"
-                       f"mcmc {mc} printfreq=100000 samplefreq=25 diagnfreq=100000 filename={d}/o;\nquit;\n")
+                       f"mcmc {mc} printfreq=100000 samplefreq=25 diagnfreq=100000 filename=o;\nquit;\n")
         report = d / "r.json"
         e = dict(os.environ, MB200_MODE="gpu", MB200_BATCH=batch, MB200_REPORT=str(report))
         e.update(env)
-        p = subprocess.run([str(BIN_BATCHED), str(nex)], cwd=ROOT, env=e, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=900)
+        p = run_mb(BIN_BATCHED, nex, e)
         assert p.returncode == 0, p.stdout[-2000:] + p.stderr[-2000:]
         rep = json.loads(report.read_text().strip().splitlines()[-1])
         rep["samples"] = {f.name: "\n".join(l for l in f.read_text().splitlines() if "ID:" not in l)
